@@ -126,6 +126,27 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_SAMPLE = 1 << 18           # --dump-outputs: elements kept per tensor (ResNet-50: 267 tensors, 35 MiB of float32)
+
+
+def dump_outputs(out_dir, loss, model):
+    """What the last timed step hands its caller: the loss ``train_step`` returned and the parameters / BatchNorm
+    statistics it left in the model, as ``<out_dir>/<name>.npy`` (float32; float64 stays float64).  A tensor of more
+    than DUMP_SAMPLE elements is flattened and sampled at positions drawn from a fixed seed, the same in every run."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss}
+    arrays.update((k, v) for k, v in model.model.state_dict().items() if v.is_floating_point() and not k.endswith(".mask"))
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
+
+
 def triangular_lr(total_steps, warmup_fraction=0.2):
     """LR multiplier schedule of the reference (utils/schedulers.py:79-117): interp [0.2, 1, 0]."""
     import numpy as np
@@ -276,7 +297,11 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="do not capture the train step into a CUDA graph")
     ap.add_argument("--no-overlap", action="store_true", help="launch the gradient exchange after the backward pass")
     ap.add_argument("--no-wgrad-side-stream", action="store_true", help="keep the weight-gradient GEMMs on the compute stream")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last timed step's loss and the "
+                    "model state it left as DIR/<name>.npy (same arguments, same inputs: compares two builds)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -296,7 +321,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
     B = args.per_gpu_batch or max(1, args.global_batch // world)
     scaling = "weak" if args.per_gpu_batch else "strong"
     use_graph = not args.no_graph
@@ -360,14 +385,19 @@ def main():
     # ---- device-resident run (value) ----
     clocks = ClockSampler(local_rank); clocks.start()
 
+    last_loss = [None]
+
     def dev_step(i):
-        loss_acc.add_(step(next(batches)))
+        last_loss[0] = step(next(batches))
+        loss_acc.add_(last_loss[0])
     ms_total = timed(K, dev_step)
     launches = launches_per_step * K
     clk = clocks.stop()
     if harness.reducer is not None:
         harness.reducer.check_status()
     img_s = world * B * K / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:             # before the eager / e2e steps below train the model further
+        dump_outputs(args.dump_outputs, last_loss[0], model)
 
     # ---- per-kernel timing of the masked GEMMs: CUDA events around every C-ABI conv call on the launching stream
     # (eager steps of the same workload through the same harness — events cannot be read back from inside a replayed graph) ----

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Generate the golden fixtures by EXECUTING THE UNMODIFIED REFERENCE (/root/reference) on CPU.
+"""Generate the golden fixtures by EXECUTING THE UNMODIFIED REFERENCE ($TURBOPRUNE_REFERENCE) on CPU.
 
 The reference has no tests / golden vectors of its own (SURVEY.md §4), so parity is pinned by
 outputs of the reference code itself, produced here once and committed:
@@ -10,8 +10,11 @@ outputs of the reference code itself, produced here once and committed:
   densities.json       generate_densities schedules
   imp_hashes.json      seed-0 ResNet-18 (CIFAR) IMP levels: SHA-256 of weights, thresholds, masks
   sgd_small.npz        torch.optim.SGD(momentum, wd) trajectory used by the reference harness
+  reference_models.json  seed-0 ResNet-18 (CIFAR) state-dict digests at init, after prune_er_erk / prune_er_balanced
+                       and after prune_mag(0.8); the reference's conf/ files the config composer is tested on
+  reference_run.npz    that model's eval logits on a fixed batch, and a batch_crop at translate = 3
 
-Run only in the build container:  python tests/golden/make_golden.py
+Run with the reference checked out:  TURBOPRUNE_REFERENCE=<dir> python tests/golden/make_golden.py
 """
 import contextlib
 import hashlib
@@ -295,7 +298,48 @@ def gen_aug():
     np.savez_compressed(os.path.join(HERE, "aug_small.npz"), **out)
 
 
+REFERENCE_CONF_FILES = [          # what compose() reads for the three compositions in test_config_composer_and_densities
+    "cifar10_er_erk.yaml", "imagenet_er_balanced.yaml",
+    "dataset_params/dp_cifar10.yaml", "optimizer_params/sgd_cifar10.yaml", "experiment_params/ep_cifar10.yaml",
+    "model_params/mp_resnet18.yaml", "dataset_params/dp_imagenet_ffcv.yaml", "optimizer_params/sgd_imagenet.yaml",
+    "experiment_params/ep_imagenet.yaml", "model_params/mp_resnet50.yaml", "cyclic_training/ct_no_cyclic.yaml",
+    "pruning_params/iterative_imp.yaml", "pruning_params/pai_er_erk.yaml", "pruning_params/iterative_wr.yaml",
+]
+
+
+def gen_reference_checks():
+    """reference_models.json / reference_run.npz: the reference's model construction, ER masks, magnitude pruning,
+    eval forward, batch_crop and conf/ tree, for the CPU tests that check the oracle and the product against them."""
+    import yaml
+    cfg = refshim.make_cfg("resnet18", "cifar10")
+    rec, run = {}, {}
+    torch.manual_seed(0)
+    r = cm.TorchVisionModel(cfg)
+    rec["init"] = refshim.state_digests(r.state_dict())
+    for fn in ("prune_er_erk", "prune_er_balanced"):
+        torch.manual_seed(5); getattr(pu, fn)(r, 0.2)
+        rec[fn] = {"state": refshim.state_digests(r.state_dict()), "sparsity_percent": r.get_overall_sparsity()}
+    torch.manual_seed(0)
+    r = cm.TorchVisionModel(cfg)
+    x = torch.randn(4, 3, 32, 32, generator=torch.Generator().manual_seed(4))
+    r.eval()
+    with torch.no_grad():
+        run["logits.x"], run["logits.y"] = x.numpy(), r(x).numpy()
+    pu.prune_mag(r, 0.8)
+    rec["prune_mag_0.8_masks"] = refshim.state_digests({n: m.mask for n, m in r.model.named_modules() if isinstance(m, (ml.ConvMask, ml.Conv1dMask, ml.LinearMask))})
+    conf = {f: yaml.safe_load(open(os.path.join(refshim.REFERENCE_ROOT, "conf", f))) for f in REFERENCE_CONF_FILES}
+    json.dump({"resnet18_cifar10": rec, "conf": conf}, open(os.path.join(HERE, "reference_models.json"), "w"), indent=0)
+
+    ds = refshim.load_reference_dataset()
+    imgs = torch.randn(5, 3, 10, 10, generator=torch.Generator().manual_seed(3))
+    pad = torch.nn.functional.pad(imgs, (3,) * 4, "reflect")                   # translate = 3
+    torch.manual_seed(8); run["crop3.out"] = ds.batch_crop(pad, 10).numpy()
+    torch.manual_seed(8); run["crop3.shifts"] = torch.randint(-3, 4, size=(5, 2)).numpy()
+    run["crop3.padded"] = pad.numpy()
+    np.savez_compressed(os.path.join(HERE, "reference_run.npz"), **run)
+
+
 if __name__ == "__main__":
-    gen_ops(); gen_prune(); gen_probs_and_hashes(); gen_densities(); gen_sgd(); gen_aug()
+    gen_ops(); gen_prune(); gen_probs_and_hashes(); gen_densities(); gen_sgd(); gen_aug(); gen_reference_checks()
     for f in sorted(os.listdir(HERE)):
         print(f, os.path.getsize(os.path.join(HERE, f)))

@@ -1,25 +1,23 @@
-"""Import the UNMODIFIED reference (/root/reference) inside the build container.
+"""Import the UNMODIFIED reference (TurboPrune, directory given by $TURBOPRUNE_REFERENCE) for fixture generation.
 
 Test/fixture infrastructure only.  The reference needs a handful of packages that
-are not in this image (fastargs, omegaconf, timm, ...); we inject empty stand-ins
-for them into ``sys.modules`` so that ``utils.mask_layers``,
+are not installed with this project (fastargs, omegaconf, timm, ...); we inject empty
+stand-ins for them into ``sys.modules`` so that ``utils.mask_layers``,
 ``utils.pruning_utils`` and ``utils.custom_models`` import unchanged.
 
-``/root/reference`` does not exist on the GPU box, so nothing under ``-m gpu``,
-``bench.py`` or ``smoke()`` may call :func:`load_reference`; it is used by
-``tests/golden/make_golden.py`` (fixture generation) and by the CPU tests that
-cross-check ``oracle/`` against the real reference when it is present.
+Only ``tests/golden/make_golden.py`` calls :func:`load_reference`: the tests compare
+against the fixtures it wrote and never need the reference itself.
 """
 import importlib
 import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("TURBOPRUNE_REFERENCE", "/root/reference")
+REFERENCE_ROOT = os.environ.get("TURBOPRUNE_REFERENCE", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "utils", "mask_layers.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "utils", "mask_layers.py"))
 
 
 def _stub(name, **attrs):
@@ -100,6 +98,16 @@ def load_reference_dataset():
         sys.modules.update(saved)
     _loaded["dataset"] = ds
     return ds
+
+
+def state_digests(state_dict):
+    """[key, dtype, shape, sha256 of the bytes] per state-dict entry: equal lists <=> bit-identical state dicts."""
+    import hashlib
+    out = []
+    for k, v in state_dict.items():
+        a = v.detach().cpu().contiguous().numpy()
+        out.append([k, str(a.dtype), list(a.shape), hashlib.sha256(a.tobytes()).hexdigest()])
+    return out
 
 
 class Cfg(dict):

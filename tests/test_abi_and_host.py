@@ -1,5 +1,6 @@
 """CPU: the C-ABI library builds for sm_100a, loads, exports every symbol the header declares; host-side
 mirrors keep the reference's surface; the product refuses to run without CUDA."""
+import json
 import os
 import re
 
@@ -8,6 +9,7 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
 def test_library_exports_every_declared_symbol(built_lib):
@@ -65,17 +67,13 @@ def test_custom_models_build_like_the_reference():
     assert m.get_overall_sparsity() == 0
     sd = m.model.state_dict()
     assert sd["fc.weight"].shape == (10, 512, 1) and sd["conv1.mask"].dtype == torch.float32
-    if refshim.reference_available():
-        ml, rpu, rcm = refshim.load_reference()
-        torch.manual_seed(0); r = rcm.TorchVisionModel(refshim.make_cfg("resnet18", "cifar10"))
-        for (k1, a), (k2, b) in zip(r.state_dict().items(), m.state_dict().items()):
-            assert k1 == k2 and torch.equal(a, b)
-        for fn in ("prune_er_erk", "prune_er_balanced"):
-            torch.manual_seed(5); getattr(pu, fn)(m, 0.2)
-            torch.manual_seed(5); getattr(rpu, fn)(r, 0.2)
-            for a, b in zip(r.state_dict().values(), m.state_dict().values()):
-                assert torch.equal(a, b)
-            assert m.get_overall_sparsity() == r.get_overall_sparsity()       # percent
+    # the reference's seed-0 model and its ER masks (tests/golden/make_golden.py): bit-identical state dicts
+    ref = json.load(open(os.path.join(GOLDEN, "reference_models.json")))["resnet18_cifar10"]
+    assert refshim.state_digests(m.state_dict()) == ref["init"]
+    for fn in ("prune_er_erk", "prune_er_balanced"):
+        torch.manual_seed(5); getattr(pu, fn)(m, 0.2)
+        assert refshim.state_digests(m.state_dict()) == ref[fn]["state"]
+        assert m.get_overall_sparsity() == ref[fn]["sparsity_percent"]       # percent
     # vgg16 / cifar100 surgery
     v = cm.TorchVisionModel(refshim.make_cfg("vgg16", "cifar100"))
     assert len(v._masked()) == 16 and v.model.state_dict()["classifier.6.weight"].shape == (100, 4096, 1)
@@ -115,7 +113,8 @@ def test_fused_sgd_state_dict_is_torch_compatible():
     assert a.param_groups[0]["lr"] == pytest.approx(0.1)
 
 
-def test_config_composer_and_densities():
+def test_config_composer_and_densities(tmp_path):
+    import yaml
     from turboprune_b200.utils import config as C
     from turboprune_b200.utils.harness_utils import generate_densities
     c = C.compose("synthetic_rn18_imp", ["experiment_params.epochs_per_level=3"], os.path.join(ROOT, "conf_b200"))
@@ -126,14 +125,17 @@ def test_config_composer_and_densities():
         C.compose("synthetic_rn18_imp", ["pruning_params.rewind_epoch=1"], os.path.join(ROOT, "conf_b200"))   # needs '+'
     c = C.compose("synthetic_rn18_imp", ["+pruning_params.rewind_epoch=1", "pruning_params=er_erk_80"], os.path.join(ROOT, "conf_b200"))
     assert c.pruning_params.prune_method == "er_erk" and c.pruning_params.rewind_epoch == 1
-    ref_conf = "/root/reference/conf"
-    if os.path.isdir(ref_conf):         # the reference's own tree, consumed unchanged (SURVEY Appendix D, configs 1-3)
-        c = C.compose("cifar10_er_erk", ["pruning_params=iterative_imp", "pruning_params.target_sparsity=0.2"], ref_conf)
-        assert generate_densities(c, 0.0) == [1.0, 0.8] and c.model_params.model_name == "resnet18"
-        c = C.compose("imagenet_er_balanced", ["pruning_params=pai_er_erk", "+pruning_params.target_sparsity=0.8"], ref_conf)
-        assert c.dataset_params.total_batch_size == 512 and generate_densities(c, 0.0) == [1 - 0.8]
-        c = C.compose("imagenet_er_balanced", ["pruning_params=iterative_wr", "pruning_params.target_sparsity=0.988"], ref_conf)
-        assert len(generate_densities(c, 0.0)) == 21
+    # the reference's own conf/ files, consumed unchanged (SURVEY Appendix D, configs 1-3), restored from the fixture
+    ref_conf = tmp_path / "conf"
+    for rel, data in json.load(open(os.path.join(GOLDEN, "reference_models.json")))["conf"].items():
+        (ref_conf / rel).parent.mkdir(parents=True, exist_ok=True)
+        (ref_conf / rel).write_text(yaml.safe_dump(data))
+    c = C.compose("cifar10_er_erk", ["pruning_params=iterative_imp", "pruning_params.target_sparsity=0.2"], str(ref_conf))
+    assert generate_densities(c, 0.0) == [1.0, 0.8] and c.model_params.model_name == "resnet18"
+    c = C.compose("imagenet_er_balanced", ["pruning_params=pai_er_erk", "+pruning_params.target_sparsity=0.8"], str(ref_conf))
+    assert c.dataset_params.total_batch_size == 512 and generate_densities(c, 0.0) == [1 - 0.8]
+    c = C.compose("imagenet_er_balanced", ["pruning_params=iterative_wr", "pruning_params.target_sparsity=0.988"], str(ref_conf))
+    assert len(generate_densities(c, 0.0)) == 21
 
 
 def test_cli_override_floats_parse_like_hydra():
