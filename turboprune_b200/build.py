@@ -17,7 +17,7 @@ NVCC_FLAGS = [
 
 
 def lib_path() -> str:
-    # TURBOPRUNE_B200_LIB: load an alternative build of the same ABI (kernel experiments: tools/build_variant.py)
+    # TURBOPRUNE_B200_LIB: load another build of the same C ABI instead (e.g. to compare two builds in one GPU run)
     return os.environ.get("TURBOPRUNE_B200_LIB") or os.path.join(LIBDIR, LIBNAME)
 
 
@@ -37,28 +37,6 @@ def _digest() -> str:
                     h.update(name.encode()); h.update(f.read())
     h.update(" ".join(NVCC_FLAGS).encode())
     return h.hexdigest()
-
-
-def build_variant(name: str, defines=()) -> str:
-    """Experiment build: the same sources with extra -D defines, linked to lib/variants/<name>.so (not the product library)."""
-    vdir = os.path.join(LIBDIR, "variants", name)
-    os.makedirs(vdir, exist_ok=True)
-    nvcc = _nvcc()
-    objs, procs = [], []
-    for src in SOURCES:
-        obj = os.path.join(vdir, src.replace(".cu", ".o"))
-        objs.append(obj)
-        cmd = [nvcc, *NVCC_FLAGS, *[f"-D{d}" for d in defines], "-c", os.path.join(CSRC, src), "-o", obj]
-        procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
-    for src, p in procs:
-        out, _ = p.communicate()
-        if p.returncode != 0:
-            raise RuntimeError(f"nvcc failed on {src}:\n{out}")
-    out = os.path.join(LIBDIR, "variants", f"{name}.so")
-    r = subprocess.run([nvcc, "-shared", "-cudart", "static", "-o", out, *objs], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-    if r.returncode != 0:
-        raise RuntimeError(f"link failed:\n{r.stdout}")
-    return out
 
 
 def build(force: bool = False, verbose: bool = True) -> str:

@@ -6,10 +6,11 @@
 // appears here as a separate pass: fprop/dgrad consume bf16 weights that were masked while
 // being staged (tp_stage_weights), wgrad applies the mask in its finalize step.
 //
-// Two persistent, warp-specialised kernels (1 CTA / SM, 192 threads):
+// Two persistent, warp-specialised kernels (1 CTA / SM):
 //   warp 0     : TMA producer (one elected lane)
 //   warp 1     : TMEM allocator + tcgen05.mma issuer (one elected lane)
-//   warps 2..5 : epilogue (TMEM -> registers -> global), one TMEM lane quarter each
+//   warps 2..  : epilogue (TMEM -> registers -> global).  fprop / dgrad: 320 threads, 8 epilogue warps, two per TMEM
+//                lane quarter; wgrad: 192 threads, 4 epilogue warps, one per quarter
 //
 //   k_igemm_fwd  : D[pixels, Cout] = A[pixels, K] * W[Cout, K]^T          (fprop, dgrad)
 //                  A tile 128 pixels x 64 channels by TMA im2col (any r,s,stride,pad) or by
@@ -32,9 +33,9 @@ constexpr int kThreads = 192;          // wgrad kernel: TMA warp, MMA warp, 4 ep
 constexpr int kFwdThreads = 320;       // fwd kernel: TMA warp, MMA warp, 8 epilogue warps (two per TMEM lane quarter)
 constexpr int kMaxTaps = 64;
 
-// smem pipeline depth of the fwd kernel: stage = A tile (16 KB) + this CTA's share of the weight tile
-__host__ __device__ constexpr int fwd_stages(int block_n, int cl) {
-  return cl == 2 ? (block_n == 256 ? 6 : 8) : (block_n == 256 ? 4 : (block_n == 128 ? 6 : 8));
+// smem pipeline depth of the fwd kernel: stage = A tile (16 KB) + weight tile (block_n x 64 bf16)
+__host__ __device__ constexpr int fwd_stages(int block_n) {
+  return block_n == 256 ? 4 : (block_n == 128 ? 6 : 8);
 }
 
 struct TapEntry { uint16_t off_w, off_h; int32_t kofs; };
@@ -51,7 +52,7 @@ struct ClsEntry {
   int ntaps, tap0;          // taps[tap0 .. tap0 + ntaps)
   int base_w, base_h;       // im2col coordinate of iteration pixel (p,q): base + q*step
   int oah, oaw;             // output pixel = (p*osh + oah, q*osw + oaw)
-  int tile0, m_groups;      // first work item of the class; M tile groups (of CL tiles) it has
+  int tile0, m_tiles;       // first work item of the class; 128-pixel M tiles it has
 };
 
 struct FwdParams {
@@ -65,10 +66,8 @@ struct FwdParams {
   int out_row_pix;          // output pixels per row
   int osh, osw;
   int linear;               // output pixel index == iteration pixel index (single class, unit output stride)
-  int ws_stages, ws_b_bytes;   // weight-stationary instantiation: activation stages, bytes of the resident weight blocks
   int ldc;                  // elements between consecutive output pixels
-  int cluster;              // thread-block cluster size along M (1 or 2): weight tile multicast
-  int tma_store;            // 1: epilogue stages 32x64 sub-tiles in smem and stores them with TMA (tmC)
+  int staged_store;         // 1 (16-byte aligned rows): the epilogue stages 32x64 sub-tiles in smem, then stores full lines
   __nv_bfloat16* out;
   const float* bias;
   const __nv_bfloat16* addend;   // optional: out = acc (+ bias) + addend[pixel][channel] (same layout as out)
@@ -87,12 +86,8 @@ struct FwdParams {
 // The staging call leaves the number of empty blocks behind the last mask row: zero (any iid unstructured mask) means
 // the K loop needs no per-block test at all.
 __device__ __forceinline__ const uint32_t* live_kmask(const uint32_t* km, int words, int N) {
-#ifdef TP_NO_KMASK          // experiment builds only: compile the skip walk out
-  return nullptr;
-#else
   if (km && __ldg(km + (size_t)((N + 63) >> 6) * words) == 0u) return nullptr;
   return km;
-#endif
 }
 
 // Which K blocks of an output-channel tile hold any non-zero weight: the OR of the occupancy words of the tile's 64-row
@@ -147,51 +142,39 @@ __device__ __forceinline__ void decompose_pixel(int m, int P, int Q, int& n, int
 }
 
 // ============================================================================================
-// CL = 1: one CTA per 128 x BLOCK_N tile (tcgen05 cta_group::1).
-// CL = 2: a CTA PAIR (cluster of 2, tcgen05 cta_group::2) works on two neighbouring M tiles of the SAME N tile as one
-// 256 x BLOCK_N UMMA: each CTA loads its own 128-pixel A tile and only HALF of the weight tile (BLOCK_N/2 rows), the
-// leader CTA's MMA thread issues the pair MMAs (they read both CTAs' shared memory), each CTA's TMEM receives its
-// own 128 rows.  L2 -> SM operand bytes per K block drop from 2 x 48 KB to 2 x 32 KB and the 32 KB stages leave room
-// for 6 of them in flight: the ncu captures showed the mainloop pinned at ~10 TB/s of L2 -> SM traffic with every
-// role waiting (profiles/r01_notes.md); TMA multicast does not reduce L2 reads at cluster size 2, operand halving does.
 struct AMaps { CUtensorMap m[kMaxCls]; };      // activation-side tensor map of every class
 
-// work item -> (class, M-tile group, N tile); identical in the three roles
-__device__ __forceinline__ void decode_tile(const FwdParams& p, int tile, int n_tiles, int& c, int& m_g, int& n_t) {
+// work item -> (class, M tile, N tile); identical in the three roles
+__device__ __forceinline__ void decode_tile(const FwdParams& p, int tile, int n_tiles, int& c, int& m_t, int& n_t) {
   c = 0;
 #pragma unroll
   for (int j = 1; j < kMaxCls; ++j) if (j < p.ncls && tile >= p.cls[j].tile0) c = j;
   const int local = tile - p.cls[c].tile0;
-  m_g = local / n_tiles; n_t = local - m_g * n_tiles;     // m-major: CTAs running together share A tiles, weights stay in L2
+  m_t = local / n_tiles; n_t = local - m_t * n_tiles;     // m-major: CTAs running together share A tiles, weights stay in L2
 }
 
+// One CTA per 128 x BLOCK_N tile, one walk over the K blocks.  A CTA-pair walk (two M tiles per UMMA, half the weight
+// tile per CTA) and a weight-stationary walk (a CTA keeps one N tile's weight blocks in smem) were built and measured
+// neutral-to-slower: the weight bytes crossing L2 -> SM do not pace these layers (profiles/r01_notes.md, r02_notes.md).
+//
 // MULTI = false: one class of output pixels (fprop, stride-1 dgrad) — the class decode, the per-row destination
 // arithmetic and the "class without taps" handling are compiled out (they cost the short-K layers up to 1.7x when they
 // sat in the common kernel: 1600 more instructions around loops that run once per 2-4 us tile).
-//
-// WS = true ("weight stationary", single class, CL = 1): when all K blocks of an output-channel tile fit in shared memory
-// next to a few activation stages (K x BLOCK_N x 2 B <= 144 KB: every 1x1 layer of ResNet-50's layer1-3, the 64-channel
-// 3x3s), a CTA keeps ONE output-channel tile for its whole life, loads its weight blocks once and then streams only
-// activation tiles.  The dense walk re-loaded BLOCK_N x 64 weights with every K block of every tile: for the 1x1 layers
-// that was 2/3 of the L2 -> SM operand traffic (128 of 192 KB per 128 x 256 x 256 tile) and it — not HBM, not the tensor
-// pipe — paced them (profiles/r01_notes.md: layer3 1x1 at 3.35 us per tile against 1.1 us of MMA and 1.9 us of HBM time).
 //
 // BNB = true (single class, linear output): the BatchNorm backward reduction of the layer that FEEDS this convolution is
 // done here, in the dgrad epilogue, instead of by k_bn_bwd_reduce (one read of dz and one of y per such layer less, one
 // launch less): after the bf16 gradient sub-tile has been staged, each lane re-reads it row-coalesced together with the
 // matching y values, applies the ReLU gate, stores g and adds sum(g), sum(g * xhat) of its 8 channels x 8 rows; rows are
 // then combined by the same fixed-order xor tree as the forward statistics.  Output: g, and [32-row group][2][N] partials.
-template <int BLOCK_N, int CL, bool MULTI, bool WS, bool BNB>
+template <int BLOCK_N, bool MULTI, bool BNB>
 __global__ void __launch_bounds__(kFwdThreads, 1)
 k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorMap tmB,
             const __grid_constant__ FwdParams p) {
-  static_assert(!WS || (CL == 1 && !MULTI), "weight-stationary walk: single CTA, single class");
-  static_assert(!BNB || (CL == 1 && !MULTI && !WS), "BatchNorm-backward epilogue: single CTA, single class, default walk");
+  static_assert(!BNB || !MULTI, "BatchNorm-backward epilogue: single class");
   constexpr int kABytes = kBlockM * kBlockK * 2;           // 16 KB
-  constexpr int kBRows = BLOCK_N / CL;                     // weight rows THIS CTA loads
-  constexpr int kBBytes = kBRows * kBlockK * 2;
+  constexpr int kBBytes = BLOCK_N * kBlockK * 2;
   constexpr int kStageBytes = kABytes + kBBytes;
-  constexpr int kStages = fwd_stages(BLOCK_N, CL);
+  constexpr int kStages = fwd_stages(BLOCK_N);
   constexpr int kAccStages = BLOCK_N == 256 ? 2 : 4;      // TMEM accumulator ring (512 columns at most)
   constexpr uint32_t kTmemCols = (kAccStages * BLOCK_N <= 32) ? 32 : (kAccStages * BLOCK_N <= 64) ? 64 :
                                  (kAccStages * BLOCK_N <= 128) ? 128 : (kAccStages * BLOCK_N <= 256) ? 256 : 512;
@@ -199,57 +182,37 @@ k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorM
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   pdl_trigger();
   constexpr int kStgBytes = 32 * 128;                      // one epilogue warp's 32 rows x 64 bf16 columns
-  constexpr int kMaxStages = 16;
-  const int n_stages = WS ? p.ws_stages : kStages;         // WS: a stage is the 16 KB activation tile alone
-  const int a_stride = WS ? kABytes : kStageBytes;
-  uint8_t* const a_base = WS ? smem + p.ws_b_bytes : smem; // WS: the resident weight blocks come first
-  uint8_t* stg_base = a_base + n_stages * a_stride;        // 4 warps x 2 buffers x 4 KB (1024-B aligned)
+  uint8_t* stg_base = smem + kStages * kStageBytes;        // 8 warps x 4 KB (1024-B aligned)
   uint64_t* full_bar = (uint64_t*)(stg_base + 8 * kStgBytes);
-  uint64_t* empty_bar = full_bar + (WS ? kMaxStages : kStages);
-  uint64_t* tfull_bar = empty_bar + (WS ? kMaxStages : kStages);
+  uint64_t* empty_bar = full_bar + kStages;
+  uint64_t* tfull_bar = empty_bar + kStages;
   uint64_t* tempty_bar = tfull_bar + kAccStages;
-  uint64_t* bres_bar = tempty_bar + kAccStages;            // WS: the resident weight blocks have landed
-  uint32_t* tmem_slot = (uint32_t*)(bres_bar + 1);
+  uint32_t* tmem_slot = (uint32_t*)(tempty_bar + kAccStages);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n_tiles = (p.N + BLOCK_N - 1) / BLOCK_N;
-  // work items are CLUSTER tiles: (class) x (group of CL neighbouring M tiles) x (N tile); CTA rank r takes M tile
-  // g*CL + r (an M tile past the end simply has no valid rows: its loads are zero-filled and its stores are masked)
-  const int cta_rank = (CL > 1) ? (int)cluster_ctarank() : 0;
-  const int cl_id = (int)blockIdx.x / CL, n_cl = (int)gridDim.x / CL;
-  const int total_tiles = p.cls[p.ncls - 1].tile0 + p.cls[p.ncls - 1].m_groups * n_tiles;
-  constexpr uint16_t kMask = (uint16_t)((1u << CL) - 1u);
-  // the w-th work item of this CTA.  WS: one fixed N tile, M tiles ws_m0, ws_m0 + ws_dm, ... (CTAs with neighbouring ids
-  // take the same M tile for the n_tiles different N tiles at about the same time: the activation tile comes from HBM once)
-  const int ws_nt = WS ? (int)blockIdx.x % n_tiles : 0;
-  const int ws_m0 = WS ? (int)blockIdx.x / n_tiles : 0, ws_dm = WS ? (int)gridDim.x / n_tiles : 1;
-  const int my_items = WS ? (p.cls[0].m_groups > ws_m0 ? (p.cls[0].m_groups - ws_m0 + ws_dm - 1) / ws_dm : 0)
-                          : (total_tiles > cl_id ? (total_tiles - cl_id + n_cl - 1) / n_cl : 0);
-  auto get_tile = [&](int w, int& ci, int& m_g, int& n_t) {
+  // work items: (class) x (M tile) x (N tile), classes back to back; CTA b takes items b, b + gridDim.x, ...
+  const int cta = (int)blockIdx.x, n_cta = (int)gridDim.x;
+  const int total_tiles = p.cls[p.ncls - 1].tile0 + p.cls[p.ncls - 1].m_tiles * n_tiles;
+  const int my_items = total_tiles > cta ? (total_tiles - cta + n_cta - 1) / n_cta : 0;
+  auto get_tile = [&](int w, int& ci, int& m_t, int& n_t) {
     ci = 0;
-    if (WS) { m_g = ws_m0 + w * ws_dm; n_t = ws_nt; return; }
-    const int tile = cl_id + w * n_cl;
-    if (MULTI) decode_tile(p, tile, n_tiles, ci, m_g, n_t);
-    else { m_g = tile / n_tiles; n_t = tile - m_g * n_tiles; }   // m-major: CTAs running together share A tiles, weights stay in L2
+    const int tile = cta + w * n_cta;
+    if (MULTI) decode_tile(p, tile, n_tiles, ci, m_t, n_t);
+    else { m_t = tile / n_tiles; n_t = tile - m_t * n_tiles; }   // m-major: CTAs running together share A tiles, weights stay in L2
   };
 
   if (warp == 0 && lane == 0) {
     for (int j = 0; j < p.ncls; ++j) prefetch_tmap(&tmA.m[j]);
     prefetch_tmap(&tmB);
-    // full / tempty are only used in the leader CTA of a pair: full gets ONE arrive (the leader's expect_tx for both
-    // CTAs' bytes), tempty gets one arrive per epilogue warp of both CTAs; empty / tfull exist in both CTAs and get
-    // one (multicast) commit arrival from the leader's MMA thread
-    for (int i = 0; i < n_stages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
-    for (int i = 0; i < kAccStages; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], 8 * CL); }
-    mbar_init(bres_bar, 1);
+    for (int i = 0; i < kStages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
+    // tempty: one arrival per epilogue warp
+    for (int i = 0; i < kAccStages; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], 8); }
     fence_mbar_init();
   }
-  if (warp == 1) {
-    if (CL == 1) { tmem_alloc(tmem_slot, kTmemCols); tmem_relinquish(); }
-    else { tmem_alloc_pair(tmem_slot, kTmemCols); tmem_relinquish_pair(); }
-  }
+  if (warp == 1) { tmem_alloc(tmem_slot, kTmemCols); tmem_relinquish(); }
   tc_fence_before();
-  if (CL > 1) cluster_sync_all(); else __syncthreads();      // peers' barriers are initialised before anyone signals them
+  __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   pdl_wait();          // barriers, TMEM and descriptor prefetch above overlap the previous grid's tail; global memory from here on
@@ -259,46 +222,25 @@ k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorM
     if (lane == 0) {
       int stage = 0; uint32_t phase = 0;
       const uint32_t* const km = live_kmask(p.kmask, p.kmask_words, p.N);
-      if (WS && my_items > 0) {
-        // every K block of this CTA's output-channel tile, once
-        const ClsEntry& c0 = p.cls[0];
-        mbar_arrive_expect_tx(bres_bar, (uint32_t)(c0.ntaps * p.cchunks * kBBytes));
-        for (int tap = 0; tap < c0.ntaps; ++tap)
-          for (int cc = 0; cc < p.cchunks; ++cc)
-            tma_load_2d(smem + (tap * p.cchunks + cc) * kBBytes, &tmB, bres_bar, p.taps[tap].kofs + cc * kBlockK, ws_nt * BLOCK_N);
-      }
       for (int w = 0; w < my_items; ++w) {
-        int ci, m_g, n_t; get_tile(w, ci, m_g, n_t);
+        int ci, m_t, n_t; get_tile(w, ci, m_t, n_t);
         const ClsEntry& ce = p.cls[MULTI ? ci : 0];
         const CUtensorMap* const mapA = &tmA.m[MULTI ? ci : 0];
-        const int m_t = m_g * CL + cta_rank;
         const int m0 = m_t * kBlockM;
         int cn = 0, cp = 0, cq = 0;
         if (p.a_mode == 1) decompose_pixel(m0, ce.P_it, ce.Q_it, cn, cp, cq);
         const int cw = ce.base_w + cq * p.step_w, ch = ce.base_h + cp * p.step_h;
         auto load_block = [&](const TapEntry& te, int cc) {
           mbar_wait(&empty_bar[stage], phase ^ 1, 1);
-          uint8_t* sA = a_base + stage * a_stride;
+          uint8_t* sA = smem + stage * kStageBytes;
           uint8_t* sB = sA + kABytes;
-          if (CL == 1) {
-            mbar_arrive_expect_tx(&full_bar[stage], WS ? kABytes : kStageBytes);
-            if (p.a_mode == 1)
-              tma_load_im2col_4d(sA, mapA, &full_bar[stage], cc * kBlockK, cw, ch, cn, te.off_w, te.off_h);
-            else
-              tma_load_2d(sA, mapA, &full_bar[stage], te.kofs + cc * kBlockK, m0);
-            if (!WS) tma_load_2d(sB, &tmB, &full_bar[stage], te.kofs + cc * kBlockK, n_t * BLOCK_N);
-          } else {
-            // pair: my A tile and my half of the weight tile land in MY shared memory, the bytes are credited to the
-            // LEADER's full barrier (which expects both CTAs' stage bytes)
-            if (cta_rank == 0) mbar_arrive_expect_tx(&full_bar[stage], kStageBytes * CL);
-            const uint32_t lead_full = mapa_u32(smem_u32(&full_bar[stage]), 0);
-            if (p.a_mode == 1)
-              tma_load_im2col_4d_pair(sA, mapA, lead_full, cc * kBlockK, cw, ch, cn, te.off_w, te.off_h);
-            else
-              tma_load_2d_pair(sA, mapA, lead_full, te.kofs + cc * kBlockK, m0);
-            tma_load_2d_pair(sB, &tmB, lead_full, te.kofs + cc * kBlockK, n_t * BLOCK_N + cta_rank * kBRows);
-          }
-          if (++stage == n_stages) { stage = 0; phase ^= 1; }
+          mbar_arrive_expect_tx(&full_bar[stage], kStageBytes);
+          if (p.a_mode == 1)
+            tma_load_im2col_4d(sA, mapA, &full_bar[stage], cc * kBlockK, cw, ch, cn, te.off_w, te.off_h);
+          else
+            tma_load_2d(sA, mapA, &full_bar[stage], te.kofs + cc * kBlockK, m0);
+          tma_load_2d(sB, &tmB, &full_bar[stage], te.kofs + cc * kBlockK, n_t * BLOCK_N);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
         };
         const int tap_base = MULTI ? ce.tap0 : 0;     // single class: a static table offset (no dependent parameter load)
         if (!km) {
@@ -326,49 +268,46 @@ k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorM
     }
   } else if (warp == 1) {
     // ------------------------------ MMA issuer ------------------------------
-    if (lane == 0 && cta_rank == 0) {
-      constexpr uint32_t idesc = make_idesc_bf16(kBlockM * CL, BLOCK_N, 0, 0);
+    if (lane == 0) {
+      constexpr uint32_t idesc = make_idesc_bf16(kBlockM, BLOCK_N, 0, 0);
       int stage = 0; uint32_t phase = 0;
       int acc = 0; uint32_t acc_phase = 0;
       const uint32_t* const km = live_kmask(p.kmask, p.kmask_words, p.N);
-      if (WS && my_items > 0) { mbar_wait(bres_bar, 0, 5); tc_fence_after(); }
       for (int w = 0; w < my_items; ++w) {
-        const int tile = cl_id + w * n_cl;      // (not used by the weight-stationary walk)
+        const int tile = cta + w * n_cta;
         if (MULTI) {      // a class no tap reaches has no accumulator: its tiles belong to the epilogue warps alone
-          int ci0, mg0, nt0; decode_tile(p, tile, n_tiles, ci0, mg0, nt0);
+          int ci0, mt0, nt0; decode_tile(p, tile, n_tiles, ci0, mt0, nt0);
           if (p.cls[ci0].ntaps == 0) continue;
         }
         mbar_wait(&tempty_bar[acc], acc_phase ^ 1, 2);
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + (uint32_t)(acc * BLOCK_N);
-        auto mma_block = [&](uint32_t accumulate, int kb) {
+        auto mma_block = [&](uint32_t accumulate) {
           mbar_wait(&full_bar[stage], phase, 3);
           tc_fence_after();
-          const uint32_t a_addr = smem_u32(a_base + stage * a_stride);
-          const uint32_t b_addr = WS ? smem_u32(smem + kb * kBBytes) : a_addr + kABytes;   // WS: K block kb of the resident tile
+          const uint32_t a_addr = smem_u32(smem + stage * kStageBytes);
+          const uint32_t b_addr = a_addr + kABytes;
           const uint64_t adesc = make_smem_desc(a_addr, 16, 1024, kLayoutSW128);
           const uint64_t bdesc = make_smem_desc(b_addr, 16, 1024, kLayoutSW128);
 #pragma unroll
           for (int k = 0; k < kBlockK / 16; ++k) {
             // advance 16 elements (32 B) along K inside the 128-B swizzle row: +2 in 16-B units
-            if (CL == 1) umma_bf16(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, accumulate | (uint32_t)k);
-            else umma_bf16_pair(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, accumulate | (uint32_t)k);
+            umma_bf16(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, accumulate | (uint32_t)k);
           }
-          // frees this smem stage (in both CTAs of a pair) when the MMAs have read it
-          if (CL == 1) umma_commit(&empty_bar[stage]); else umma_commit_pair(&empty_bar[stage], kMask);
-          if (++stage == n_stages) { stage = 0; phase ^= 1; }
+          umma_commit(&empty_bar[stage]);        // frees this smem stage when the MMAs have read it
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
         };
         if (!MULTI && !km) {
           // dense single-class walk: no tile arithmetic at all on this thread (it paces the tensor pipe)
           const int kiters = p.cls[0].ntaps * p.cchunks;
-          for (int it = 0; it < kiters; ++it) mma_block((uint32_t)it, it);
+          for (int it = 0; it < kiters; ++it) mma_block((uint32_t)it);
         } else {
-          int ci = 0, m_g = 0, n_t = 0;
-          if (MULTI) decode_tile(p, tile, n_tiles, ci, m_g, n_t); else n_t = WS ? ws_nt : tile % n_tiles;
+          int ci = 0, m_t = 0, n_t = 0;
+          if (MULTI) decode_tile(p, tile, n_tiles, ci, m_t, n_t); else n_t = tile % n_tiles;
           const ClsEntry& ce = p.cls[MULTI ? ci : 0];       // a class without taps issues nothing: its epilogue writes the addend (or zero) alone
           if (!km) {
             const int kiters = ce.ntaps * p.cchunks;
-            for (int it = 0; it < kiters; ++it) mma_block((uint32_t)it, it);
+            for (int it = 0; it < kiters; ++it) mma_block((uint32_t)it);
           } else {
             KSkip ks; uint32_t any = 0;
             ks.begin(km, p.kmask_words, n_t * BLOCK_N, BLOCK_N, p.N);
@@ -377,14 +316,13 @@ k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorM
               for (int cc = 0; cc < p.cchunks; ++cc) {
                 const bool last = tap == ce.ntaps - 1 && cc == p.cchunks - 1;
                 if (!ks.on(kb0 + cc) && !(last && !any)) continue;               // same decision as the producer
-                mma_block(any, tap * p.cchunks + cc);
+                mma_block(any);
                 any = 1;
               }
             }
           }
         }
-        // accumulator complete -> epilogue (of both CTAs of a pair)
-        if (CL == 1) umma_commit(&tfull_bar[acc]); else umma_commit_pair(&tfull_bar[acc], kMask);
+        umma_commit(&tfull_bar[acc]);            // accumulator complete -> epilogue
         if (++acc == kAccStages) { acc = 0; acc_phase ^= 1; }
       }
     }
@@ -396,14 +334,13 @@ k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorM
     const int half = (warp - 2) >> 2;         // which half of the 64-column chunks this warp drains
     int acc = 0; uint32_t acc_phase = 0;
     for (int w = 0; w < my_items; ++w) {
-      int ci, m_g, n_t; get_tile(w, ci, m_g, n_t);
+      int ci, m_t, n_t; get_tile(w, ci, m_t, n_t);
       const ClsEntry& ce = p.cls[MULTI ? ci : 0];
       const bool has_acc = MULTI ? ce.ntaps > 0 : true;   // a class no tap reaches: the accumulator was never written, its value is zero
-      const int m_t = m_g * CL + cta_rank;
       const int row = m_t * kBlockM + quarter * 32 + lane;
       const bool row_ok = row < ce.M;
       long long opix = 0;
-      if (row_ok && !p.tma_store) {       // generic output mapping, one division chain per tile
+      if (row_ok && !p.staged_store) {    // generic output mapping, one division chain per tile
         opix = row;
         if (MULTI || !p.linear) {
           int n, pp, qq; decompose_pixel(row, ce.P_it, ce.Q_it, n, pp, qq);
@@ -421,7 +358,7 @@ k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorM
       // the destination pixel — ONE division chain for the first row, the other seven follow by stepping 4 pixels
       long long ooff[MULTI ? 8 : 1];
       const long long rbase = (wrow0 + r_in) * ldc + c16 * 8;
-      if (MULTI && p.tma_store) {
+      if (MULTI && p.staged_store) {
         int n, pp, qq; decompose_pixel((int)(wrow0 + r_in), ce.P_it, ce.Q_it, n, pp, qq);
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
@@ -435,7 +372,7 @@ k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorM
       if (MULTI && !has_acc) {
         // parity class no tap reaches (e.g. 3 of the 4 classes of a 1x1 stride-2 convolution): dX there is the fused addend
         // or zero — plain coalesced copies / stores; no accumulator exists, so no hand-shake with the MMA thread either
-        if (p.tma_store) {
+        if (p.staged_store) {
 #pragma unroll 1
           for (int c = half * 64; c < BLOCK_N; c += 128) {
             const int n0 = n_t * BLOCK_N + c;
@@ -460,7 +397,7 @@ k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorM
       mbar_wait(&tfull_bar[acc], acc_phase, 4);
       tc_fence_after();
       const uint32_t t_base = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BLOCK_N);
-      if (p.tma_store) {
+      if (p.staged_store) {
         // TMEM -> registers -> 128B-swizzled smem sub-tile (32 rows x 64 cols) -> coalesced global
         // stores, so every output line leaves the SM as full 128-byte rows instead of 32 scattered 16-byte pieces.
         // Everything that does not depend on the column chunk is hoisted (row pointers, validity, swizzled
@@ -682,19 +619,13 @@ k_igemm_fwd(const __grid_constant__ AMaps tmA, const __grid_constant__ CUtensorM
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if (CL == 1) mbar_arrive(&tempty_bar[acc]);
-        else mbar_arrive_cluster(mapa_u32(smem_u32(&tempty_bar[acc]), 0));     // the leader's MMA thread owns the accumulators
-      }
+      if (lane == 0) mbar_arrive(&tempty_bar[acc]);
       if (++acc == kAccStages) { acc = 0; acc_phase ^= 1; }
     }
   }
   tc_fence_before();
-  if (CL > 1) cluster_sync_all(); else __syncthreads();      // nobody exits while the pair may still touch its smem / TMEM
-  if (warp == 1) {
-    tc_fence_after();
-    if (CL == 1) tmem_dealloc(tmem_base, kTmemCols); else tmem_dealloc_pair(tmem_base, kTmemCols);
-  }
+  __syncthreads();
+  if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem_base, kTmemCols); }
 }
 
 // ============================================================================================
@@ -1095,49 +1026,27 @@ static int pick_block_n(long long m_tiles, int n) {
   return best;
 }
 
-constexpr int kSmemMax = 232448;                 // 227 KB: the per-CTA opt-in limit of sm_100
-constexpr int kWsMaxBBytes = 144 * 1024;         // resident weight blocks of the weight-stationary walk
-
-template <int BN, int CL, bool MULTI, bool WS, bool BNB = false>
+template <int BN, bool MULTI, bool BNB = false>
 static int launch_fwd(const AMaps& a, const CUtensorMap& b, FwdParams& p, cudaStream_t st) {
-  constexpr int kStages = fwd_stages(BN, CL);
   constexpr int kTail = 8 * 32 * 128 + 1024 + 512;    // epilogue staging, alignment slack, barriers
-  int smem = kStages * (kBlockM * kBlockK * 2 + (BN / CL) * kBlockK * 2) + kTail;
+  constexpr int smem = fwd_stages(BN) * (kBlockM * kBlockK * 2 + BN * kBlockK * 2) + kTail;
   const int n_tiles = (p.N + BN - 1) / BN;
-  if (WS) {
-    p.ws_b_bytes = p.cls[0].ntaps * p.cchunks * BN * kBlockK * 2;
-    p.ws_stages = (kSmemMax - kTail - p.ws_b_bytes) / (kBlockM * kBlockK * 2);
-    if (p.ws_stages > 16) p.ws_stages = 16;
-    if (p.ws_stages < 3) return TP_ERR_UNSUPPORTED;
-    smem = p.ws_b_bytes + p.ws_stages * kBlockM * kBlockK * 2 + kTail;
-  }
   static bool attr_set = false;
   if (!attr_set) {
-    TP_CUDA_CHECK(cudaFuncSetAttribute(k_igemm_fwd<BN, CL, MULTI, WS, BNB>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS ? kSmemMax : smem));
+    TP_CUDA_CHECK(cudaFuncSetAttribute(k_igemm_fwd<BN, MULTI, BNB>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     attr_set = true;
   }
-  // work items: per class, (groups of CL M tiles) x (N tiles), classes back to back
+  // work items: per class, (M tiles) x (N tiles), classes back to back
   long long ctiles = 0;
   for (int c = 0; c < p.ncls; ++c) {
-    const long long m_tiles = (p.cls[c].M + kBlockM - 1) / kBlockM;
-    p.cls[c].m_groups = (int)((m_tiles + CL - 1) / CL);
+    p.cls[c].m_tiles = (int)((p.cls[c].M + kBlockM - 1) / kBlockM);
     if (ctiles > 0x7fffffffll) return TP_ERR_UNSUPPORTED;
     p.cls[c].tile0 = (int)ctiles;
-    ctiles += (long long)p.cls[c].m_groups * n_tiles;
+    ctiles += (long long)p.cls[c].m_tiles * n_tiles;
   }
   if (ctiles > 0x7fffffffll || ctiles <= 0) return TP_ERR_UNSUPPORTED;
-  const long long max_cl = sm_count() / CL;
-  int grid = (int)(ctiles < max_cl ? ctiles : max_cl) * CL;
-  if (WS) grid = (sm_count() / n_tiles) * n_tiles;           // every CTA owns one N tile: a whole number of CTAs per N tile
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kFwdThreads); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = (CL == 1 && pdl_enabled()) ? 2 : 1;     // pairs stay fully serialised
-  TP_CUDA_CHECK(cudaLaunchKernelEx(&cfg, k_igemm_fwd<BN, CL, MULTI, WS, BNB>, a, b, p));
+  const int grid = (int)(ctiles < sm_count() ? ctiles : sm_count());
+  TP_CUDA_CHECK(launch(k_igemm_fwd<BN, MULTI, BNB>, grid, kFwdThreads, smem, st, a, b, p));
   TP_LAUNCH_CHECK();
   return TP_OK;
 }
@@ -1147,65 +1056,25 @@ static int run_fwd(const AMaps& a, const CUtensorMap& b, FwdParams& p, int bn, c
   // (for any pixel mapping: a strided dgrad's parity classes compute the destination pixel of each row)
   p.linear = p.ncls == 1 && p.osh == 1 && p.osw == 1 && p.cls[0].oah == 0 && p.cls[0].oaw == 0 &&
              p.out_row_pix == p.cls[0].Q_it && p.out_img_pix == (long long)p.cls[0].P_it * p.cls[0].Q_it;
-  p.tma_store = (p.ldc % 8 == 0 && p.N % 8 == 0 && (((uintptr_t)p.out) & 15) == 0 &&
-                 (!p.addend || (((uintptr_t)p.addend) & 15) == 0)) ? 1 : 0;
-  if (p.stats && !(p.tma_store && p.linear)) return TP_ERR_UNSUPPORTED;
+  p.staged_store = (p.ldc % 8 == 0 && p.N % 8 == 0 && (((uintptr_t)p.out) & 15) == 0 &&
+                    (!p.addend || (((uintptr_t)p.addend) & 15) == 0)) ? 1 : 0;
+  if (p.stats && !(p.staged_store && p.linear)) return TP_ERR_UNSUPPORTED;
   // the general-mapping instantiation only where it is needed: parity classes, or a single class whose output is not
   // the iteration order itself
-  const bool multi = !p.linear;
-  if (multi) {
-    if (p.cluster == 2) {
-      if (bn == 256) return launch_fwd<256, 2, true, false>(a, b, p, st);
-      if (bn == 128) return launch_fwd<128, 2, true, false>(a, b, p, st);
-      return launch_fwd<64, 2, true, false>(a, b, p, st);
-    }
-    if (bn == 256) return launch_fwd<256, 1, true, false>(a, b, p, st);
-    if (bn == 128) return launch_fwd<128, 1, true, false>(a, b, p, st);
-    return launch_fwd<64, 1, true, false>(a, b, p, st);
-  }
-  if (p.cluster == 2) {
-    if (bn == 256) return launch_fwd<256, 2, false, false>(a, b, p, st);
-    if (bn == 128) return launch_fwd<128, 2, false, false>(a, b, p, st);
-    return launch_fwd<64, 2, false, false>(a, b, p, st);
+  if (!p.linear) {
+    if (bn == 256) return launch_fwd<256, true>(a, b, p, st);
+    if (bn == 128) return launch_fwd<128, true>(a, b, p, st);
+    return launch_fwd<64, true>(a, b, p, st);
   }
   if (p.bn_y) {      // BatchNorm-backward epilogue (needs the linear staged path; the caller checked the shapes)
-    if (!p.tma_store || !p.stats) return TP_ERR_UNSUPPORTED;
-    if (bn == 256) return launch_fwd<256, 1, false, false, true>(a, b, p, st);
-    if (bn == 128) return launch_fwd<128, 1, false, false, true>(a, b, p, st);
-    return launch_fwd<64, 1, false, false, true>(a, b, p, st);
+    if (!p.staged_store || !p.stats) return TP_ERR_UNSUPPORTED;
+    if (bn == 256) return launch_fwd<256, false, true>(a, b, p, st);
+    if (bn == 128) return launch_fwd<128, false, true>(a, b, p, st);
+    return launch_fwd<64, false, true>(a, b, p, st);
   }
-  // weight-stationary walk: the tile's weight blocks fit next to >= 3 activation stages, there is a whole number of CTAs
-  // per N tile and enough M tiles for every CTA to amortise the one-time weight load
-  const int n_tiles = (p.N + bn - 1) / bn;
-  const long long m_tiles = (p.cls[0].M + kBlockM - 1) / kBlockM;
-  const long long b_bytes = (long long)p.cls[0].ntaps * p.cchunks * bn * kBlockK * 2;
-  // Measured on B200 (profiles/r02_notes.md, conv_bench at B = 512): bit-identical, but only 0-5 % faster on the layer3
-  // 1x1s and 5-8 % SLOWER on layer1's (fewer bytes in flight per SM with 16 KB stages) — like the cta_group::2 pair kernel
-  // of round 1 this says the weight bytes crossing L2 -> SM are not what paces these layers.  Opt-in (TP_IGEMM_WS=1),
-  // parity-tested.
-  const char* e = getenv("TP_IGEMM_WS");
-  const bool ws = e && atoi(e) != 0 && b_bytes <= kWsMaxBBytes && n_tiles <= sm_count() / 2 && m_tiles >= 4ll * (sm_count() / n_tiles);
-  if (ws) {
-    if (bn == 256) return launch_fwd<256, 1, false, true>(a, b, p, st);
-    if (bn == 128) return launch_fwd<128, 1, false, true>(a, b, p, st);
-    return launch_fwd<64, 1, false, true>(a, b, p, st);
-  }
-  if (bn == 256) return launch_fwd<256, 1, false, false>(a, b, p, st);
-  if (bn == 128) return launch_fwd<128, 1, false, false>(a, b, p, st);
-  return launch_fwd<64, 1, false, false>(a, b, p, st);
-}
-
-// Cluster size for a problem: pairs of M tiles share the weight tile (multicast) whenever there are enough tiles.
-static int pick_cluster(long long m_tiles) {
-  const char* e = getenv("TP_IGEMM_CLUSTER");        // read every call: the parity tests flip it
-  const int forced = e ? atoi(e) : 0;
-  if (forced == 1 || forced == 2) return forced;
-  // Measured on B200 (profiles/r01_notes.md, tools/conv_bench.py): the cta_group::2 pair kernel is bit-identical but
-  // not faster — 0.92-0.96x on the layer4 GEMMs, 1.05-1.4x SLOWER on the HBM-bound layers (both CTAs' epilogues and
-  // loads gate every accumulator hand-off through cluster-remote arrivals).  The mainloop is not L2-bandwidth bound,
-  // the per-tile epilogue is.  Pairs stay selectable with TP_IGEMM_CLUSTER=2 (parity-tested).
-  (void)m_tiles;
-  return 1;
+  if (bn == 256) return launch_fwd<256, false>(a, b, p, st);
+  if (bn == 128) return launch_fwd<128, false>(a, b, p, st);
+  return launch_fwd<64, false>(a, b, p, st);
 }
 
 }  // namespace tp
@@ -1281,8 +1150,7 @@ int tp_conv_fprop_stats(const tp_conv_desc* d, const void* x, const void* wf, co
   }
   for (int c = 1; c < kMaxCls; ++c) ta.m[c] = ta.m[0];
   const int bn = pick_block_n((p.M + kBlockM - 1) / kBlockM, p.N);
-  p.cluster = pick_cluster((p.M + kBlockM - 1) / kBlockM);
-  rc = make_tiled_map(&tb, wf, (uint64_t)d->r * d->s * d->cin, (uint64_t)d->cout, (uint64_t)d->r * d->s * d->cin, (uint32_t)(bn / p.cluster));
+  rc = make_tiled_map(&tb, wf, (uint64_t)d->r * d->s * d->cin, (uint64_t)d->cout, (uint64_t)d->r * d->s * d->cin, (uint32_t)bn);
   if (rc) return rc;
   return run_fwd(ta, tb, p, bn, st);
 }
@@ -1401,8 +1269,7 @@ static int conv_dgrad_impl(const tp_conv_desc* d, const void* dy, const void* wd
   long long m_tiles = 0;
   for (int c = 0; c < p.ncls; ++c) m_tiles += (p.cls[c].M + kBlockM - 1) / kBlockM;
   const int bn = pick_block_n(m_tiles, p.N);
-  p.cluster = pick_cluster(m_tiles);
-  rc = make_tiled_map(&tb, wd, (uint64_t)ktot, (uint64_t)d->cin, (uint64_t)ktot, (uint32_t)(bn / p.cluster)); if (rc) return rc;
+  rc = make_tiled_map(&tb, wd, (uint64_t)ktot, (uint64_t)d->cin, (uint64_t)ktot, (uint32_t)bn); if (rc) return rc;
   return run_fwd(ta, tb, p, bn, st);
 }
 

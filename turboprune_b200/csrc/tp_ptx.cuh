@@ -18,9 +18,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void fence_mbar_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
-__device__ __forceinline__ void fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
@@ -78,46 +75,6 @@ __device__ __forceinline__ void tma_load_im2col_4d(void* dst, const CUtensorMap*
       : "memory");
 }
 
-// CTA-pair (cta_group::2) variants: the box lands in THIS CTA's shared memory, the transaction bytes are credited
-// to an mbarrier of the pair's leader CTA (`lead_bar` is a shared::cluster address, see mapa_u32).
-__device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* map, uint32_t lead_bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      :: "r"(smem_u32(dst)), "l"(map), "r"(lead_bar), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tma_load_im2col_4d_pair(void* dst, const CUtensorMap* map, uint32_t lead_bar,
-                                                        int c, int w, int h, int n, uint16_t off_w, uint16_t off_h) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.im2col.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5, %6}], [%2], {%7, %8};"
-      :: "r"(smem_u32(dst)), "l"(map), "r"(lead_bar), "r"(c), "r"(w), "r"(h), "r"(n), "h"(off_w), "h"(off_h)
-      : "memory");
-}
-// shared::cluster address of `addr` (a shared::cta address of this CTA) in the CTA with cluster rank `rank`
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t addr, uint32_t rank) {
-  uint32_t r; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank)); return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" :: "r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
-// smem -> global tile store (coalesced full lines; clips at the tensor bounds)
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-               :: "l"(map), "r"(smem_u32(src)), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" :: "n"(N) : "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
 // ---- tcgen05 / TMEM ----------------------------------------------------------------------
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(dst_smem)), "r"(ncols) : "memory");
@@ -127,16 +84,6 @@ __device__ __forceinline__ void tmem_relinquish() {
 }
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(taddr), "r"(ncols) : "memory");
-}
-// CTA-pair TMEM management: the same warp of BOTH CTAs issues these (same shared-memory slot offset in both)
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t* dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(dst_smem)), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_pair() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" :: "r"(taddr), "r"(ncols) : "memory");
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after()  { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
@@ -153,21 +100,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t adesc, uint6
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
                :: "r"(smem_u32(bar)) : "memory");
-}
-// CTA-pair MMA (issued by one thread of the LEADER CTA): M = 256 rows, 128 from each CTA's A tile; each CTA supplies
-// N/2 rows of B; each CTA's TMEM receives its own 128 rows x N columns.  Descriptors are the leader's shared-memory
-// offsets (the peer uses the same offsets).
-__device__ __forceinline__ void umma_bf16_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      :: "r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-// Pair commit: arrives on the barrier at this offset in every CTA of `cta_mask` once the pair's MMAs have completed.
-__device__ __forceinline__ void umma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               :: "r"(smem_u32(bar)), "h"(cta_mask) : "memory");
 }
 // TMEM -> registers: 32 lanes x 32 columns of 32-bit; thread i of the warp gets lane (base+i).
 __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t* v) {
@@ -186,7 +118,7 @@ __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.
 // ---- descriptors ---------------------------------------------------------------------------
 // Shared-memory matrix descriptor (cute::UMMA::SmemDescriptor bit layout): start address,
 // leading-dim and stride-dim byte offsets in 16-byte units, version 1, layout type in [61,64).
-constexpr uint32_t kLayoutNone = 0, kLayoutSW128 = 2;
+constexpr uint32_t kLayoutSW128 = 2;
 __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t layout) {
   return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) |
          ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
@@ -199,16 +131,6 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr, uint32_t 
 __host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N, int a_major, int b_major) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_major << 15) | ((uint32_t)b_major << 16) |
          ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile(
-      "{\n\t.reg .pred P;\n\t"
-      "elect.sync _|P, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, P;\n\t}"
-      : "=r"(pred) :: "memory");
-  return pred != 0;
 }
 
 }}  // namespace tp::ptx
