@@ -163,6 +163,20 @@ int tp_im2col_stem(const void* src, int src_dtype, int64_t sn, int64_t sc, int64
 int tp_cifar_augment(const void* src, void* out, const int64_t* shifts, const uint8_t* flip,
                      const int64_t* cut_y, const int64_t* cut_x, int cut_size,
                      int n, int c, int h, int w, int r, void* stream);
+/* tp_cifar_epoch: one epoch of CifarLoader.__iter__ (utils/dataset.py:192-226) straight from the data set as stored,
+ * src uint8 [n][h][w][c] (c <= 4, h*w*c <= 20 KiB), into out fp32 [n][c][h][w] contiguous and labels_out int64 [n]:
+ *   i = perm ? perm[j] : j;  x1 = (flip_all || flip[i]) ? w-1-x : x;  yy = refl(y + shifts[i][0]);  xx = refl(x1 + shifts[i][1])
+ *   xx = preflip[i] ? w-1-xx : xx;   out[j][ch][y][x] = inside_cut(i,y,x) ? 0 : (src[i][yy][xx][ch] * (1/255) - mean[ch]) / std[ch]
+ *   labels_out[j] = labels[i]
+ * refl(-1) = 1, refl(h) = h-2 (F.pad reflect); each arithmetic step rounds once, as torch's separate CUDA kernels do.
+ * Every array but src / out is optional: perm int64 [n] (NULL: identity), shifts int64 [n][2] in [-r, r] with 0 < r < h, w
+ * (NULL: no translate), preflip / flip uint8 [n] (NULL: none; flip_all != 0 flips every image and excludes flip),
+ * cut_y / cut_x int64 [n] corners of a cut_size square (both NULL: none), labels / labels_out (both or neither).
+ * mean / std are HOST arrays of c floats.  All NULL: the normalised set in stored order (the test loader). */
+int tp_cifar_epoch(const uint8_t* src, const int64_t* labels, void* out, int64_t* labels_out, const int64_t* perm,
+                   const int64_t* shifts, int r, const uint8_t* preflip, const uint8_t* flip, int flip_all,
+                   const int64_t* cut_y, const int64_t* cut_x, int cut_size, const float* mean, const float* std,
+                   int n, int c, int h, int w, void* stream);
 /* Synthetic batches (stand-in for the FFCV / CIFAR loaders, which need data sets): Philox4x32-10, counter
  * (counter_offset + i/4, 0, 0, 0), key = seed; element i takes word i%4.  tp_synth_normal writes N(0,1) fp32 (Box-Muller
  * on 24-bit uniforms; raw_words != 0: the 32-bit words themselves, for bit-exact pinning of the stream);

@@ -55,6 +55,8 @@ SIGNATURES = {
     "tp_im2col_c8": (c_int, [c_void_p] + [c_int] * 11 + [c_void_p, c_int, c_void_p]),
     "tp_im2col_stem": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_int64] + [c_int] * 13 + [c_void_p, c_int, c_void_p]),
     "tp_cifar_augment": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "tp_cifar_epoch": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int,
+                               c_void_p, c_void_p, c_int, POINTER(c_float), POINTER(c_float), c_int, c_int, c_int, c_int, c_void_p]),
     "tp_synth_normal": (c_int, [c_void_p, c_int64, c_uint64, c_uint64, c_int, c_void_p]),
     "tp_synth_labels": (c_int, [c_void_p, c_int64, c_int, c_uint64, c_uint64, c_void_p]),
     "tp_conv_workspace_bytes": (c_size_t, [POINTER(ConvDesc), c_int]),

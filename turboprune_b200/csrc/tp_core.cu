@@ -104,7 +104,7 @@ const char* tp_strerror(int code) {
 }
 
 const char* tp_last_cuda_error(void) { return tp::g_last_err; }
-int tp_abi_version(void) { return 8; }
+int tp_abi_version(void) { return 9; }
 int tp_device_sm_count(void) { return tp::sm_count(); }
 int tp_set_pdl(int on) { const int prev = tp::pdl_enabled() ? 1 : 0; tp::g_pdl = on ? 1 : 0; return prev; }
 

@@ -3,8 +3,10 @@
 ``PruningHarness(cfg, gpu_id, expt_dir, model=None)`` and ``.train_one_level(epochs_per_level, level)`` keep the
 reference's behaviour (:28-50, :159-269): a fresh optimizer and LR schedule per level (momentum never carries
 over), ``model_init.pt`` / ``optimizer_init.pt`` at level 0, ``model_rewind.pt`` at ``pruning_params.rewind_epoch``,
-per-level CSV + summary CSV.  Optimizer = ``FusedSGD`` (same state-dict layout as torch.optim.SGD), loaders = the
-synthetic on-device generator (the real loaders are out of scope).
+per-level CSV + summary CSV.  Optimizer = ``FusedSGD`` (same state-dict layout as torch.optim.SGD).  Loaders =
+``utils.dataset.make_loaders``: the CIFAR data set under ``dataset_params.data_root_dir`` (``AirbenchLoaders``) when a
+CIFAR config sets ``dataset_params.dataloader_type`` to anything but ``synthetic``, as the reference's configs do
+(``torch``); otherwise, and for ImageNet, the synthetic on-device generator.
 """
 import csv
 import os
@@ -16,7 +18,7 @@ import torch.nn as nn
 from ..optim import FusedSGD
 from ..utils import schedulers
 from ..utils.custom_models import CustomModel, TorchVisionModel
-from ..utils.dataset import SyntheticLoaders
+from ..utils.dataset import make_loaders
 from ..utils.harness_utils import save_model
 from .base_harness import BaseHarness
 
@@ -44,7 +46,7 @@ class PruningHarness(BaseHarness):
     def _setup_dataloaders(self):
         world = torch.distributed.get_world_size() if self.distributed else 1
         rank = torch.distributed.get_rank() if self.distributed else 0
-        loaders = SyntheticLoaders(self.cfg, self.device, world, rank)
+        loaders = make_loaders(self.cfg, self.device, world, rank)
         return loaders.train_loader, loaders.test_loader
 
     def _setup_optimizer(self):
